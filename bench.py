@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native Discregrid hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Metric (BASELINE.json): "SDF grid nodes/sec (addFunction) + interpolate Mqueries/sec".
@@ -27,22 +27,29 @@ The second half of the metric, interpolate()+gradient Mqueries/s (config 4: 10 M
 under "interpolate" and nested in roofline / e2e / cpu_baseline (the driver keeps those objects whole).
 """
 import argparse
+import atexit
 import ctypes as C
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the source tree (no __pycache__ either)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 WORKLOAD = {"source": "bunny", "resolution": [128, 128, 128], "torus": (186, 187, 1.0, 0.4, 0.05, 7, 5)}
 INTERP = {"resolution": [256, 256, 256], "queries": 10_000_000, "seed": 0x5EED}
-RES_DIR = os.path.join(ROOT, "oracle", "_ref", "resources")      # the reference's meshes (inputs), staged by `make -C oracle ref`
+# --dump-outputs: 2^21 of the headline grid's nodes (16 MB) and 2^20 of the interpolate queries (phi + gradient, 32 MB)
+DUMP = {"sdf_nodes": 1 << 21, "queries": 1 << 20, "seed": 0xD1F}
+# the reference's meshes (inputs), staged by `make -C oracle ref`; DG_BENCH_MESH_DIR points elsewhere (the CPU rehearsal stages small stand-ins)
+RES_DIR = os.environ.get("DG_BENCH_MESH_DIR") or os.path.join(ROOT, "oracle", "_ref", "resources")
 
 
 def parse():
@@ -67,22 +74,42 @@ def parse():
     ap.add_argument("--no-real", action="store_true", help="skip the leg on the other reference meshes (dragon / happy_buddha)")
     ap.add_argument("--no-density", action="store_true", help="skip the density-map (K3) legs (diagnostics / profiling)")
     ap.add_argument("--cpu-seconds", type=float, default=40.0, help="a CPU leg whose full-size run is estimated to take longer than this falls back to a strided sample")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what they computed as DIR/<name>.npy (float64; fixed seeded samples of the large arrays)")
     ap.add_argument("--cpu-child", default="", help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.sharding == "auto":
         args.sharding = "interleaved" if int(os.environ.get("WORLD_SIZE", "1")) >= 4 else "chunks"
     return args
 
 
 # ------------------------------------------------------------------------------------------------ helpers
+_SCRATCH = []
+
+
 def scratch_dir():
-    """for the few hundred MB some legs exchange through files: the repo's own volume (build/ is git-ignored); /tmp can be a slow copy-on-write layer"""
-    d = os.path.join(ROOT, "build")
-    try:
-        os.makedirs(d, exist_ok=True)
-        return d
-    except OSError:
-        return "/tmp"
+    """for the few hundred MB some legs exchange through files: a private temporary directory, removed at exit (the source tree may be
+    read-only, and the benchmark leaves nothing in it)"""
+    if not _SCRATCH:
+        _SCRATCH.append(tempfile.mkdtemp(prefix="dg_bench_"))
+        atexit.register(shutil.rmtree, _SCRATCH[0], True)
+    return _SCRATCH[0]
+
+
+def dump_sample(n, k, seed):
+    """--dump-outputs: a fixed, seeded, sorted sample of k of the indices 0..n-1 (all of them when n <= k)"""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: every array as <path>/<name>.npy in float64"""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, np.float64))
 
 
 def workload_mesh(dg, source, torus=None):
@@ -492,6 +519,12 @@ def main():
     launches = (dg.kernel_launch_count() - launches0) * args.steps // (args.steps + args.warmup)
     sharded_ok = same_as_single_launch(md, desc, n_nodes, full)
     clocks = sampler.stop() if rank == 0 else None
+    dumped = {}
+    if args.dump_outputs and rank == 0:
+        # the coefficients of the last timed step, before any later leg reuses `full`
+        idx = torch.from_numpy(dump_sample(n_nodes, DUMP["sdf_nodes"], DUMP["seed"])).to(dev)
+        dumped["sdf_nodes"] = full[idx].cpu().numpy()
+        del idx
     ms_step = float(np.mean(sdf_ms))
     value = n_nodes / (ms_step * 1e-3)
 
@@ -625,6 +658,11 @@ def main():
         xd = xd_keep
         del xd_sorted
         interp_step(True); torch.cuda.synchronize()          # phi / grad hold the unsorted queries' results again (compared with the host path below)
+        if args.dump_outputs and rank == 0:
+            qi = torch.from_numpy(dump_sample(q_hi - q_lo, DUMP["queries"], DUMP["seed"])).to(dev)
+            dumped["interpolate_phi"] = phi[qi].cpu().numpy()
+            dumped["interpolate_grad"] = grad[qi].cpu().numpy()
+            del qi
         alg = 312.0 * (q_hi - q_lo)
         gbs = alg / (ig_ms * 1e-3) / 1e9
         # e2e through the host API: page-locked host buffers (the contract's pinned inputs), H2D + kernel + D2H inside the timed region
@@ -886,6 +924,8 @@ def main():
                                                          "interpolate_queries_compared": ((interp or {}).get("cpu_baseline") or {}).get("queries_compared")},
                 "sharded_equals_single_launch": sharded_ok,
                 "library": {"path": os.path.relpath(capi.LIB_PATH, ROOT), "emulated": hasattr(capi.lib, "emu_mesh_create")}}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -1,5 +1,5 @@
-"""Regenerates the committed golden fixtures.  Run in the build container (needs /root/reference and
-oracle/_ref/libdgref.so = the reference's own unmodified TriangleMeshDistance.h, built by `make -C oracle ref`):
+"""Regenerates the committed golden fixtures.  Run where the reference is compiled: `make -C oracle ref REF=<checkout of the
+reference>` builds oracle/_ref (libdgref.so = its own unmodified TriangleMeshDistance.h, its grid class and tools) and stages its meshes:
 
     python tests/golden/make_golden.py
 
@@ -10,18 +10,20 @@ Outputs (all small, committed):
                              points around a deterministic 4,608-triangle bumpy torus (discregrid_b200.mesh.bumpy_torus)
   ref_torus_tree.npz         the reference's tree (children + internal spheres) and pseudonormals for that torus
   ref_sphere_surface.npz     reference results for points ON / very near a UV sphere's surface (ties, sign near 0)
+  ref_digests.json           sha256 digests of the reference's results where the arrays would be too large to commit
+                             (oracle_api.ref_check): the tests that compare with the reference on generated inputs are run
+                             with DG_RECORD_REF_DIGESTS=1 at the end of this script
 """
-import os, shutil, sys
+import json, os, shutil, sys
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
-from oracle_api import RefMesh, Oracle          # noqa: E402
+from oracle_api import REF_DIGESTS, REF_RESOURCES as REF_RES, RefMesh, Oracle, digest   # noqa: E402
 import ctypes as C                             # noqa: E402
 from discregrid_b200.mesh import bumpy_torus, uv_sphere   # noqa: E402 (pure numpy part of the package)
 
-REF_RES = "/root/reference/cmd/generate_sdf/resources"
 for f in ("box.obj", "box.cdf"):
     shutil.copyfile(os.path.join(REF_RES, f), os.path.join(HERE, f))
     os.chmod(os.path.join(HERE, f), 0o644)
@@ -101,11 +103,23 @@ for tag, path, fields in (("box", "box.cdf", (0,)), ("red", "ref_sphere_reduced.
         out[f"{tag}_f{f}_phi_only"] = g.interpolate(f, xq, grad=False)[0]
     if tag == "box":
         ok, N, dN, c0, cells, phi2, grad2 = g.split(0, xq[:1500])
-        out.update(box_split_ok=ok, box_split_N=N, box_split_dN=dN, box_split_c0=c0, box_split_cell=cells, box_split_phi=phi2, box_split_grad=grad2)
+        out.update(box_split_ok=ok, box_split_c0=c0, box_split_cell=cells, box_split_phi=phi2, box_split_grad=grad2)
+        # the shape functions and their gradients (1500 x 32 x 4 doubles) would take the file past 1 MB: kept as a digest
+        digests = json.load(open(REF_DIGESTS)) if os.path.exists(REF_DIGESTS) else {}
+        digests["ref_grid_queries/box_split_N_dN"] = digest((N[ok.astype(bool)], dN[ok.astype(bool)]), nan_equal=False)
+        with open(REF_DIGESTS, "w") as f:
+            json.dump(digests, f, indent=0, sort_keys=True)
+            f.write("\n")
 np.savez_compressed(os.path.join(HERE, "ref_grid_queries.npz"), **out)
 
 # reduceField on an ANISOTROPIC grid: cells of 1/6 x 1/3 x 2/3 make several surviving nodes share one Morton key (the key's cell
 # size is the largest one, :1114), so the node order of the result depends on how std::sort leaves equal keys -- the case
 # dg_reduce_field handles by replaying the reference's own sort.  Input and the reference's output are both committed.
 subprocess.run([sys.executable, os.path.join(HERE, "make_reduce_golden.py")], check=True)
+
+# digests of the reference's results on the inputs the tests generate (oracle_api.ref_check): the tests record them themselves
+subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", "-m", "not gpu", "-k",
+                "awkward or non_finite or fuzz or against_the_reference_library or real_addfunction",
+                "tests/test_k1_emulated.py", "tests/test_k23_emulated.py", "tests/test_reduce_field.py", "tests/test_oracle_reference_tools.py"],
+               cwd=ROOT, env=dict(os.environ, DG_RECORD_REF_DIGESTS="1"), check=True)
 print("golden fixtures written to", HERE)

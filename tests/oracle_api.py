@@ -2,6 +2,8 @@
 TriangleMeshDistance.h (oracle/_ref/libdgref.so).  TEST INFRASTRUCTURE ONLY -- the product package
 (discregrid_b200/) never imports this module."""
 import ctypes as C
+import hashlib
+import json
 import os
 import numpy as np
 
@@ -11,6 +13,7 @@ REF_SO = os.path.join(ROOT, "oracle", "_ref", "libdgref.so")
 REF_RESOURCES = os.path.join(ROOT, "oracle", "_ref", "resources")
 REF_GRID_SO = os.path.join(ROOT, "oracle", "_ref", "libdiscregrid_ref.so")
 REF_BIN = os.path.join(ROOT, "oracle", "_ref", "bin")
+REF_DIGESTS = os.path.join(ROOT, "tests", "golden", "ref_digests.json")
 
 _dp = C.POINTER(C.c_double)
 _u32p = C.POINTER(C.c_uint32)
@@ -28,6 +31,52 @@ def _f64(a):
 
 def _u32(a):
     return np.ascontiguousarray(a, dtype=np.uint32)
+
+
+def digest(arrays, nan_equal=True):
+    """sha256 over a tuple of arrays (length and values; integers as int64, floats as float64).  nan_equal: every NaN is replaced by
+    the same NaN first, so that two results have the same digest exactly when they are equal bit for bit, any NaN matching any NaN."""
+    h = hashlib.sha256()
+    for a in arrays:
+        a = np.asarray(a).ravel()
+        if a.dtype.kind == "f":
+            a = a.astype(np.float64)
+            if nan_equal:
+                a = np.where(np.isnan(a), np.nan, a)
+        else:
+            a = a.astype(np.int64)
+        h.update(b"%d:" % len(a))
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+_digests = None
+
+
+def ref_check(key, got, live, nan_equal=True):
+    """True when `got` (a tuple of arrays) equals the reference's result on the same inputs.  The reference's results on the test inputs are
+    kept as digests in tests/golden/ref_digests.json, so that the comparison needs no build of the reference.  `live` computes the result
+    with the reference itself (oracle/_ref); it runs instead when `key` is not stored, and DG_RECORD_REF_DIGESTS=1 makes it run and store its
+    digest under `key` (tests/golden/make_golden.py).  live=None: the stored digest only (written by make_golden.py itself)."""
+    global _digests
+    if _digests is None:
+        _digests = json.load(open(REF_DIGESTS)) if os.path.exists(REF_DIGESTS) else {}
+    record = os.environ.get("DG_RECORD_REF_DIGESTS") == "1"
+    if key in _digests and (not record or live is None):
+        return digest(got, nan_equal) == _digests[key]
+    if live is None:
+        raise KeyError(f"no stored digest of the reference's result for {key!r}")
+    try:
+        want = digest(live(), nan_equal)
+    except OSError as ex:
+        raise KeyError(f"no stored digest of the reference's result for {key!r}, and the reference is not built (oracle/_ref)") from ex
+    if record:
+        _digests = json.load(open(REF_DIGESTS)) if os.path.exists(REF_DIGESTS) else {}
+        _digests[key] = want
+        with open(REF_DIGESTS, "w") as f:
+            json.dump(_digests, f, indent=0, sort_keys=True)
+            f.write("\n")
+    return digest(got, nan_equal) == want
 
 
 class _MeshBase:

@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN, ROOT, bits_equal
+from oracle_api import ref_check
 from test_oracle_golden import read_cdf
 from test_oracle_reference_tools import split_inputs
 
@@ -105,7 +106,7 @@ def test_shape_function_kernel_matches_reference_class(dg):
     xi = np.ascontiguousarray(xi)
     N = np.empty((len(xi), 32)); dN = np.empty((len(xi), 32, 3))
     capi.check(capi.lib.dg_shape_functions(capi.ptr(xi, capi.F64P), len(xi), capi.ptr(N, capi.F64P), capi.ptr(dN, capi.F64P)))
-    assert bits_equal(N, q["box_split_N"][ok]) and bits_equal(dN, q["box_split_dN"][ok])
+    assert ref_check("ref_grid_queries/box_split_N_dN", (N, dN), None, nan_equal=False)
 
 
 def test_python_reduce_field_then_interpolate(dg):

@@ -64,14 +64,21 @@ def test_smoke_entry_point_on_the_emulated_library():
     assert r.returncode == 0 and "smoke OK" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
 
 
-def test_bench_runs_end_to_end_single_rank():
+def test_bench_runs_end_to_end_single_rank(tmp_path):
     """bench.py, every leg, at toy sizes (tests/emu/bench_rehearsal.py: torch's CUDA surface on host stand-ins, emulated kernels): one JSON
     line with the contract's keys; the legs that self-check (interpolate / density vs the CPU references, reduceField vs the reference
-    class) report agreement"""
+    class) report agreement.  The reference-mesh leg runs on a small stand-in (tests/golden/sphere.obj staged as dragon.obj), and
+    --dump-outputs writes the sampled outputs of the timed steps"""
+    import shutil
+    import numpy as np
     if not os.path.exists(EMU):
         pytest.skip("build/bin/libdgemu.so not built (make cpp)")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "emu", "bench_rehearsal.py")] + TOY, cwd=ROOT,
-                       env=dict(os.environ, DISCREGRID_B200_LIB=EMU, DG_ALLOW_EMULATED_LIBRARY="1"), capture_output=True, text=True, timeout=1200)
+    meshes, out = tmp_path / "meshes", tmp_path / "out"
+    meshes.mkdir()
+    shutil.copy(os.path.join(ROOT, "tests", "golden", "sphere.obj"), meshes / "dragon.obj")
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "emu", "bench_rehearsal.py")] + TOY + ["--dump-outputs", str(out)], cwd=ROOT,
+                       env=dict(os.environ, DISCREGRID_B200_LIB=EMU, DG_ALLOW_EMULATED_LIBRARY="1", DG_BENCH_MESH_DIR=str(meshes)),
+                       capture_output=True, text=True, timeout=1200)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-3000:]
     d = _bench_line(r.stdout)
     for key in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline", "dtype", "data", "config",
@@ -81,6 +88,10 @@ def test_bench_runs_end_to_end_single_rank():
     assert {"bound", "achieved", "peak", "unit", "frac", "traffic"} <= set(d["roofline"]) and {"value", "unit", "cores", "kind", "sample"} <= set(d["cpu_baseline"])
     assert d["interpolate"]["cpu_baseline"]["bit_exact_vs_gpu"] is True
     assert d["target_config"]["value"] > 0 and len(d["reference_meshes"]) >= 1
+    dumped = {p.name: np.load(p) for p in out.iterdir()}
+    assert set(dumped) == {"sdf_nodes.npy", "interpolate_phi.npy", "interpolate_grad.npy"}
+    assert all(a.dtype == np.float64 and np.isfinite(a).all() for a in dumped.values())
+    assert len(dumped["sdf_nodes.npy"]) == d["config"]["nodes"] and dumped["interpolate_grad.npy"].shape == (len(dumped["interpolate_phi.npy"]), 3)
     red = d["density_map"]["reduce_field"]
     assert "error" not in red and red["nodes_out"] > 0
     if "reference" in red:

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN, bits_equal
+from oracle_api import ref_check
 from test_oracle_golden import read_cdf, read_obj
 
 DBL_MAX = np.finfo(np.float64).max
@@ -95,7 +96,7 @@ def test_split_api_matches_reference_class(orc):
     c0, xi, mi = split_inputs(g, x[ok])
     assert bits_equal(c0, q["box_split_c0"][ok])
     N, dN = orc.shape_functions(xi)
-    assert bits_equal(N, q["box_split_N"][ok]) and bits_equal(dN, q["box_split_dN"][ok])      # shape_function_ pinned to the reference's code
+    assert ref_check("ref_grid_queries/box_split_N_dN", (N, dN), None, nan_equal=False)       # shape_function_ pinned to the reference's code
     cell_id = g["res"][1] * g["res"][0] * mi[:, 2] + g["res"][0] * mi[:, 1] + mi[:, 0]
     assert np.array_equal(g["cells"][0][cell_id], q["box_split_cell"][ok])
     assert bits_equal(q["box_split_phi"][ok], q["box_f0_phi"][:1500][ok]) and bits_equal(q["box_split_grad"][ok], q["box_f0_grad"][:1500][ok])
@@ -123,18 +124,15 @@ def test_real_meshes_through_reference_tool(orc, mesh, fixture, sign):
 def test_oracle_equals_the_references_real_addfunction(orc):
     """refg_add_function_sdf drives the reference's own CubicLagrangeDiscreteGrid::addFunction with the GenerateSDF functor
     (cubic_lagrange_discrete_grid.cpp:780-899; cmd/generate_sdf/main.cpp:92-105): node coefficients, connectivity table and node count
-    equal the oracle's restatement bit for bit -- also inverted and on an anisotropic resolution"""
-    from oracle_api import RefAddFunction, have_ref_grid
-    if not have_ref_grid():
-        pytest.skip("oracle/_ref/libdiscregrid_ref.so not built")
+    equal the oracle's restatement bit for bit -- also inverted and on an anisotropic resolution (the reference's results stored as
+    digests, oracle_api.ref_check)"""
+    from oracle_api import RefAddFunction
     import discregrid_b200 as dg
     t = dg.bumpy_torus(30, 24, 1.0, 0.4, 0.05, 7, 5)
-    ref = RefAddFunction(t.vertices, t.faces)
     mesh = orc.mesh(t.vertices, t.faces)
     mn, mx = orc.generate_sdf_domain(t.vertices)
     for res, invert in (((9, 7, 5), False), ((6, 6, 6), True)):
-        dt, nodes, cells = ref.add_function(mn, mx, res, invert=invert, want_nodes=True, want_cells=True)
         gd, r = orc.grid_desc(mn, mx, res)
         want = mesh.sample_sdf(gd, r, sign=-1.0 if invert else 1.0)
-        assert dt > 0 and np.array_equal(nodes.view(np.uint64), want.view(np.uint64))
-        assert np.array_equal(cells, orc.build_cells(r))
+        reference = lambda: RefAddFunction(t.vertices, t.faces).add_function(mn, mx, res, invert=invert, want_nodes=True, want_cells=True)[1:]
+        assert ref_check(f"ref_add_function/torus30x24/{res}/invert={invert}", (want, orc.build_cells(r)), reference, nan_equal=False)

@@ -116,21 +116,22 @@ def test_facade_reduce_field_glue_without_gpu(dg, tmp_path):
 @pytest.mark.parametrize("mn,mx,res,lo,hi", [([-1, -1, -1], [1, 1, 1], (16, 16, 16), 0.5, 0.7), ([-1, -2, -1], [1, 1, 3], (20, 9, 14), 0.5, 1.2),
                                              ([0, 0, 0], [1, 2, 4], (5, 7, 3), 0.0, 5.0), ([-1, -1, -1], [1, 1, 1], (40, 40, 40), 0.55, 0.7)])
 def test_against_the_reference_library(dg, orc, tmp_path, mn, mx, res, lo, hi):
-    """where the reference itself was compiled (oracle/_ref): random blob fields reduced by the reference class and by dg_reduce_field"""
-    from oracle_api import REF_GRID_SO, RefGrid
-    if not os.path.exists(REF_GRID_SO):
-        pytest.skip("oracle/_ref/libdiscregrid_ref.so not built (needs /root/reference)")
+    """random blob fields reduced by dg_reduce_field and by the reference class (its results stored as digests, oracle_api.ref_check)"""
+    from oracle_api import RefGrid, ref_check
     import sys
     sys.path.insert(0, GOLDEN)
     from make_reduce_golden import synthetic_field, write_cdf
     gd, r, v, cells = synthetic_field(orc, mn, mx, res, 7)
     src = str(tmp_path / "in.cdf")
     write_cdf(src, mn, mx, res, gd[6:9], gd[9:12], v, cells, np.arange(len(cells), dtype=np.uint32))
-    ref = RefGrid(src); ref.reduce_window(0, lo, hi); ref.save(str(tmp_path / "out.cdf")); ref.close()
-    want = read_cdf(str(tmp_path / "out.cdf"))
+
+    def reference():
+        ref = RefGrid(src); ref.reduce_window(0, lo, hi); ref.save(str(tmp_path / "out.cdf")); ref.close()
+        want = read_cdf(str(tmp_path / "out.cdf"))
+        return want["nodes"][0], want["cells"][0], want["cmap"][0]
     g = dict(mn=np.array(mn, float), mx=np.array(mx, float), res=np.array(res, np.uint32), cell=gd[6:9], inv=gd[9:12])
     nodes, c2, cmap = reduce_field(dg, g, v, (lo <= v) & (v <= hi) & (v != DBL_MAX), cells)
-    assert bits_equal(nodes, want["nodes"][0]) and np.array_equal(c2, want["cells"][0]) and np.array_equal(cmap, want["cmap"][0])
+    assert ref_check(f"reduce_field/{mn}/{mx}/{res}/{lo}/{hi}", (nodes, c2, cmap), reference, nan_equal=False)
 
 
 def test_threaded_sort_replay_equals_std_sort():

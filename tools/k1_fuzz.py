@@ -5,12 +5,13 @@ triangles, cubes / octahedra with queries on symmetry planes, duplicated triangl
 distance bits, nearest point, entity and triangle id.  usage: tools/k1_fuzz.py [rounds=200] [seed=0] [lib=libk1emu.so] [points|grid]
 mode `grid` runs the addFunction NODE LOOP (sdf_sample_nodes_kernel: bricks of lattice nodes, the packet walk when built with K1_PACKET) on
 lattices laid over the same meshes -- half-integer lattices through the symmetric ones -- and compares sign * distance bit for bit with the
-reference header evaluated at the node positions."""
+reference header evaluated at the node positions.  The reference's results come from tests/golden/ref_digests.json where they are stored
+for a case (oracle_api.ref_check), from oracle/_ref otherwise; a mismatch is reported per case."""
 import ctypes as C, os, sys
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
-from oracle_api import RefMesh
+from oracle_api import RefMesh, ref_check
 rounds = int(sys.argv[1]) if len(sys.argv) > 1 else 200
 seed = int(sys.argv[2]) if len(sys.argv) > 2 else 0
 so = sys.argv[3] if len(sys.argv) > 3 else os.path.join(ROOT, "build", "bin", "libk1emu.so")
@@ -79,10 +80,6 @@ bad = 0
 total = 0
 for k in range(rounds):
     V, F, x = make_case(k)
-    try:
-        ref = RefMesh(V, F)
-    except Exception as ex:
-        print("reference refused the mesh", ex); continue
     h = lib.emu_mesh_create(V.ctypes.data_as(dp), len(V), F.ctypes.data_as(u32p), len(F))
     if mode == "grid":
         from oracle_api import Oracle
@@ -95,29 +92,24 @@ for k in range(rounds):
         nn = (res[0] + 1) * (res[1] + 1) * (res[2] + 1) + 2 * (res[0] * (res[1] + 1) * (res[2] + 1) + (res[0] + 1) * res[1] * (res[2] + 1) + (res[0] + 1) * (res[1] + 1) * res[2])
         xs = np.empty((nn, 3)); lib.emu_node_positions(gd.ctypes.data_as(dp), r.ctypes.data_as(u32p), 0, nn, xs.ctypes.data_as(dp))
         sign = 1.0 if k % 2 else -1.0
-        wd = ref.distance(xs, signed=True)[0]
-        want = wd if sign == 1.0 else sign * wd
         got = np.full(nn, np.nan)
         assert lib.emu_sample_sdf(h, gd.ctypes.data_as(dp), r.ctypes.data_as(u32p), sign, 0, nn, got.ctypes.data_as(dp)) == 0
-        ok = (got.view(np.uint64) == want.view(np.uint64)) | (np.isnan(got) & np.isnan(want))
         total += nn
-        if not ok.all():
-            i = int(np.nonzero(~ok)[0][0]); bad += int((~ok).sum())
-            print(f"MISMATCH case {k} (kind {k % 7}, {len(F)} tris) grid {res} node {i} x={xs[i]!r}: {got[i]!r} vs {want[i]!r}")
+        key = f"k1_fuzz/grid/{seed}/{k}"
+        if not ref_check(key, (got,), lambda: (sign * RefMesh(V, F).distance(xs, signed=True)[0],)):
+            bad += 1
+            print(f"MISMATCH {key} (kind {k % 7}, {len(F)} tris) grid {res}")
         lib.emu_mesh_destroy(h)
         continue
     n = len(x)
     for signed in (1, 0):
-        wd, wn, we, wt = ref.distance(x, signed=bool(signed))
         d = np.zeros(n); nr = np.zeros((n, 3)); e = np.zeros(n, np.int32); t = np.zeros(n, np.int32)
         lib.emu_mesh_distance(h, x.ctypes.data_as(dp), n, signed, d.ctypes.data_as(dp), nr.ctypes.data_as(dp), e.ctypes.data_as(i32p), t.ctypes.data_as(i32p))
-        okd = (d.view(np.uint64) == wd.view(np.uint64)) | (np.isnan(d) & np.isnan(wd))
-        okn = ((nr.view(np.uint64) == wn.view(np.uint64)) | (np.isnan(nr) & np.isnan(wn))).all(1)
-        ok = okd & okn & (e == we) & (t == wt)
         total += n
-        if not ok.all():
-            i = int(np.nonzero(~ok)[0][0]); bad += int((~ok).sum())
-            print(f"MISMATCH case {k} (kind {k % 7}, {len(F)} tris) signed={signed} x={x[i]!r}: d {d[i]!r} vs {wd[i]!r}, tri {t[i]} vs {wt[i]}, ent {e[i]} vs {we[i]}")
+        key = f"k1_fuzz/points/{seed}/{k}/signed={signed}"
+        if not ref_check(key, (d, nr, e, t), lambda: RefMesh(V, F).distance(x, signed=bool(signed))):
+            bad += 1
+            print(f"MISMATCH {key} (kind {k % 7}, {len(F)} tris)")
     lib.emu_mesh_destroy(h)
-print(f"{rounds} meshes, {total} queries, {bad} mismatches")
+print(f"{rounds} meshes, {total} queries, {bad} mismatches (result sets that differ from the reference)")
 sys.exit(1 if bad else 0)

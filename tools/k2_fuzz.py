@@ -2,16 +2,21 @@
 """Parity fuzzer (CPU) for interpolate: the product's K2 kernel code run by tests/emu (build/bin/libk23emu.so) against the reference's own
 CubicLagrangeDiscreteGrid::interpolate (oracle/_ref/libdiscregrid_ref.so) on random grids (anisotropic, offset, tiny / huge cells), random
 fields with DBL_MAX sentinels, optionally reduced, and queries that sit on cell faces, domain corners and outside, plus NaN / infinities:
-value + gradient and value-only, bit for bit.  usage: tools/k2_fuzz.py [rounds=60] [seed=0]"""
+value + gradient and value-only, bit for bit.  The reduced fields are made by the product's dg_reduce_field (host passes) and checked against
+the reference's reduceField first.  The reference's results come from tests/golden/ref_digests.json where they are stored for a case
+(oracle_api.ref_check), from oracle/_ref otherwise; a mismatch is reported per case.  usage: tools/k2_fuzz.py [rounds=60] [seed=0]"""
 import ctypes as C, os, sys, tempfile
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests")); sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-from oracle_api import Oracle, RefGrid
+from oracle_api import Oracle, RefGrid, ref_check
 from make_reduce_golden import write_cdf
 from test_oracle_golden import read_cdf
+from test_reduce_field import reduce_field
+import discregrid_b200 as dg
 rounds = int(sys.argv[1]) if len(sys.argv) > 1 else 60
-rng = np.random.default_rng(int(sys.argv[2]) if len(sys.argv) > 2 else 0)
+seed = int(sys.argv[2]) if len(sys.argv) > 2 else 0
+rng = np.random.default_rng(seed)
 lib = C.CDLL(os.path.join(ROOT, "build", "bin", "libk23emu.so"))
 dp, u32p = C.POINTER(C.c_double), C.POINTER(C.c_uint32)
 lib.emu_field_create.restype = C.c_void_p
@@ -32,13 +37,26 @@ for k in range(rounds):
     n = int(cells.max()) + 1
     v = rng.standard_normal(n) * 10.0 ** rng.integers(-3, 4)
     if k % 3 == 1: v[rng.random(n) < 0.05] = DBL_MAX                 # missing coefficients
-    src = os.path.join(tmp, "in.cdf")
+    src, dst = os.path.join(tmp, "in.cdf"), os.path.join(tmp, "reduced.cdf")
     write_cdf(src, mn, mx, res, gd[6:9], gd[9:12], v, cells, np.arange(len(cells), dtype=np.uint32))
-    ref = RefGrid(src)
-    if k % 3 == 2:                                                    # a reduced field: removed cells, renumbered nodes
-        ref.reduce_window(0, float(np.quantile(v, 0.3)), float(np.quantile(v, 0.7))); ref.save(src)
-        ref.close(); ref = RefGrid(src)
     g = read_cdf(src)
+    field = (g["nodes"][0], g["cells"][0], g["cmap"][0])
+
+    def ref_grid():
+        ref = RefGrid(src)
+        if k % 3 == 2:
+            ref.reduce_window(0, lo, hi); ref.save(dst); ref.close(); ref = RefGrid(dst)
+        return ref
+    if k % 3 == 2:                                                    # a reduced field: removed cells, renumbered nodes
+        lo, hi = float(np.quantile(v, 0.3)), float(np.quantile(v, 0.7))
+        field = reduce_field(dg, g, v, (lo <= v) & (v <= hi) & (v != DBL_MAX), cells)
+
+        def ref_reduced():
+            ref_grid().close(); r_ = read_cdf(dst)
+            return r_["nodes"][0], r_["cells"][0], r_["cmap"][0]
+        if not ref_check(f"k2_fuzz/{seed}/{k}/reduced", field, ref_reduced, nan_equal=False):
+            bad += 1
+            print(f"MISMATCH k2_fuzz/{seed}/{k}/reduced: dg_reduce_field differs from the reference's reduceField")
     ext = mx - mn
     xs = [mn - 0.1 * ext + rng.random((400, 3)) * 1.2 * ext]
     faces = [mn[d] + gd[6 + d] * np.arange(res[d] + 1) for d in range(3)]
@@ -47,20 +65,21 @@ for k in range(rounds):
     xs.append(np.array([mn, mx, [mn[0], mx[1], mn[2]], 0.5 * (mn + mx), np.nextafter(mx, np.inf), np.nextafter(mn, -np.inf),
                         [np.nan, mn[1], mn[2]], [np.inf, mn[1], mn[2]], [mn[0], -np.inf, mn[2]], [0.0, 0.0, 0.0], [-0.0, -0.0, -0.0]]))
     x = np.ascontiguousarray(np.concatenate(xs)); m = len(x)
-    want_phi, want_grad = ref.interpolate(0, x, grad=True)
-    want_only = ref.interpolate(0, x, grad=False)[0]
-    ref.close()
-    nodes = np.ascontiguousarray(g["nodes"][0]); cc = np.ascontiguousarray(g["cells"][0], np.uint32); cm = np.ascontiguousarray(g["cmap"][0], np.uint32)
+
+    def ref_interpolate():
+        ref = ref_grid()
+        want = ref.interpolate(0, x, grad=True) + (ref.interpolate(0, x, grad=False)[0],)
+        ref.close()
+        return want
+    nodes = np.ascontiguousarray(field[0]); cc = np.ascontiguousarray(field[1], np.uint32); cm = np.ascontiguousarray(field[2], np.uint32)
     h = lib.emu_field_create(gd.ctypes.data_as(dp), r.ctypes.data_as(u32p), nodes.ctypes.data_as(dp), cc.ctypes.data_as(u32p), len(cc), cm.ctypes.data_as(u32p))
     phi = np.zeros(m); grad = np.zeros((m, 3)); only = np.zeros(m)
     lib.emu_interpolate(h, x.ctypes.data_as(dp), m, phi.ctypes.data_as(dp), grad.ctypes.data_as(dp))
     lib.emu_interpolate(h, x.ctypes.data_as(dp), m, only.ctypes.data_as(dp), None)
     lib.emu_field_destroy(h)
-    same = lambda a, b: (a.view(np.uint64) == b.view(np.uint64)) | (np.isnan(a) & np.isnan(b))
-    ok = same(phi, want_phi) & same(grad, want_grad).all(1) & same(only, want_only)
     total += m
-    if not ok.all():
-        i = int(np.nonzero(~ok)[0][0]); bad += int((~ok).sum())
-        print(f"MISMATCH case {k} res {res} x={x[i]!r}: phi {phi[i]!r} vs {want_phi[i]!r}, grad {grad[i]} vs {want_grad[i]}, value-only {only[i]!r} vs {want_only[i]!r}")
-print(f"{rounds} fields, {total} queries, {bad} mismatches")
+    if not ref_check(f"k2_fuzz/{seed}/{k}", (phi, grad, only), ref_interpolate):
+        bad += 1
+        print(f"MISMATCH k2_fuzz/{seed}/{k} res {res}")
+print(f"{rounds} fields, {total} queries, {bad} mismatches (result sets that differ from the reference)")
 sys.exit(1 if bad else 0)
